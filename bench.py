@@ -13,6 +13,10 @@ The steps are PIPELINED over `--depth` lanes of one context (include/ualm.h: sev
 while the slowest trajectories of step s still run, and every step's results are complete inside the timed region.  `value` is
 measured with the problems resident in HBM; `e2e` goes through the host-buffer C-ABI calls (ualm_submit_batch / ualm_wait_batch)
 with pinned host inputs, H2D and D2H inside the timed region.  One JSON line on stdout (rank 0).
+
+--dump-outputs DIR writes what the headline path returned in its last timed step (rank 0's shard): the coefficient vectors
+c_xy / c_yaw and one array per result field, float64 .npy files, a fixed seeded sample of trajectories when they exceed 64 MB.
+The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -27,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ next to the sources
 
 METRIC = "converged trajectories/sec (batch MINCO)"
 UNIT = "traj/s"
@@ -214,6 +219,32 @@ def time_reference_build(m, params, pb, threads, nprob=16):
             "note": "bit-identical to the oracle port (tests/test_ref_pin.py); slower only because the Eigen stand-in is eager"}
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, res, cxy, cyaw, pb):
+    """DIR/<name>.npy of one solved batch: c_xy, c_yaw and every ualm_result_t field, all float64.  Over DUMP_LIMIT bytes, a fixed seeded
+    sample of whole trajectories is written instead, with their problem indices in sample_index.npy."""
+    from uneven_planner_b200 import api
+    fields = [f for f, _ in api.Result._fields_ if f != "reserved"]
+    per = 8 * (12 * pb.N.astype(np.int64) + 6 * pb.M.astype(np.int64) + len(fields) + 1)
+    idx = np.arange(pb.B)
+    if per.sum() > DUMP_LIMIT:
+        order = np.random.default_rng(0).permutation(pb.B)
+        idx = np.sort(order[np.cumsum(per[order]) <= DUMP_LIMIT])
+    _, _, ocx, ocy = pb.offsets()
+    out = {"c_xy": np.concatenate([cxy[ocx[i]:ocx[i + 1]] for i in idx]) if len(idx) else np.zeros(0),
+           "c_yaw": np.concatenate([cyaw[ocy[i]:ocy[i + 1]] for i in idx]) if len(idx) else np.zeros(0)}
+    for f in fields:
+        out[f] = np.array([getattr(res[i], f) for i in idx], dtype=np.float64)
+    if len(idx) < pb.B:
+        out["sample_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+    note("wrote %d arrays of %d trajectories to %s" % (len(out), len(idx), path))
+
+
 def cpu_parallel_run(po, params, m, pb, threads):
     """the oracle on `threads` host threads over pb: (converged/s, seconds, converged count, mean in-thread seconds per trajectory)"""
     t0 = time.perf_counter()
@@ -267,7 +298,7 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=8)
+    ap.add_argument("--steps", type=int, default=8, help="timed steps of every timed region (the throughput path's 8 lanes want 24 or more)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4, 5], help="BASELINE.json config number (1-based)")
@@ -283,6 +314,8 @@ def main():
     ap.add_argument("--ref-sample", type=int, default=0, dest="ref_sample", help="reference arm / cpu_baseline: problems per step (0 = the whole batch, bounded at 1024 for cpu_baseline)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the un-pipelined latency datapoint and the penalty-kernel timing")
+    ap.add_argument("--dump-outputs", default="", dest="dump_outputs", metavar="DIR",
+                    help="write the results of the last timed step of the headline path to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -321,7 +354,7 @@ def main():
     host_in = [k[1] for k in keep]
     h2d = int(sum(a.nbytes for a in host_in))
 
-    def measure(precision, depth, steps, warmup, with_clocks):
+    def measure(precision, depth, steps, warmup, with_clocks, dump=False):
         """`value` (problems resident in HBM, steps pipelined over `depth` lanes) and `e2e` (host buffers through ualm_submit_batch /
         ualm_wait_batch) of one context of the given precision.  Returns a dict; the context stays open in r["opt"]."""
         opt = api.BatchALMTrajOpt(device=local_rank, precision=precision).init(params).set_environment(m)
@@ -373,6 +406,10 @@ def main():
         if world > 1:
             dist.all_reduce(tms, op=dist.ReduceOp.MAX)
         ms = float(tms.item())
+        last = None
+        if dump:
+            opt.select_lane((steps - 1) % depth)
+            last = opt.download()
         opt.select_lane(0)
         _, launches = opt.last_solve_ms()
         res, cxy, cyaw = opt.download()
@@ -398,7 +435,7 @@ def main():
                 r, _, _ = opt.wait(tickets[s], out=outs[s % depth][:3])
                 conv += sum(1 for q in r if q.ret_code == 0)
             return conv
-        e2e_steps = max(depth, min(steps, 2 * depth))
+        e2e_steps = steps
         note("precision %d: value done (%.1f ms/step), e2e" % (precision, ms / steps))
         run_e2e(depth)
         barrier()
@@ -413,7 +450,7 @@ def main():
             e2e_s, conv_e2e = float(tmax[0].item()), float(te[1].item())
         d2h = int(C.sizeof(api.Result) * pb.B + outs[0][1].nbytes + outs[0][2].nbytes)
         return dict(opt=opt, ms=ms, lanes_ms=lanes_ms, value=conv_total * steps / (ms * 1e-3), conv_total=conv_total, conv_local=conv_local,
-                    res=res, launches=launches, clocks=clocks, depth=depth, steps=steps,
+                    res=res, last=last, launches=launches, clocks=clocks, depth=depth, steps=steps,
                     e2e={"value": conv_e2e / e2e_s, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "steps": e2e_steps,
                          "api": "ualm_submit_batch / ualm_wait_batch, pinned host buffers, %d batches in flight" % depth})
 
@@ -434,7 +471,9 @@ def main():
     # ---------------- the headline: the parity path (precision 64, bit-identical to the oracle) ----------------
     head_prec = args.precision
     depth = max(1, min(args.depth if args.depth > 0 else (3 if head_prec == 64 else 8), 8))
-    r0 = measure(head_prec, depth, args.steps, args.warmup, True)
+    r0 = measure(head_prec, depth, args.steps, args.warmup, True, dump=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *r0["last"], pb)
     opt, res, ms, lanes_ms, value, conv_total, conv_local, launches, clocks = (r0[k] for k in ("opt", "res", "ms", "lanes_ms", "value", "conv_total", "conv_local", "launches", "clocks"))
     opt.select_lane(0)
     quality = quality_of(opt, res)
@@ -498,9 +537,9 @@ def main():
     fast = None
     if head_prec == 64 and not args.no_fast:
         fdepth = 8
-        # three pipeline lengths of timed steps: the timed region starts and ends with an empty pipeline (synchronize on both sides), so a short one
-        # mostly measures filling and draining the eight lanes
-        rf = measure(32, fdepth, max(2 * args.steps, 3 * fdepth), max(args.warmup, fdepth), False)
+        # the timed region starts and ends with an empty pipeline (synchronize on both sides), so fewer steps than about three times the
+        # eight lanes mostly measure filling and draining them
+        rf = measure(32, fdepth, args.steps, max(args.warmup, fdepth), False)
         fo = rf["opt"]
         fo.select_lane(0)
         note("fast path measured; post-solve scan")
@@ -513,7 +552,10 @@ def main():
                                          "holds the end-to-end distribution)" % ROUND,
                 "value": rf["value"], "solved_per_s": Btot * rf["steps"] / (rf["ms"] * 1e-3), "unit": UNIT, "ms_per_step": rf["ms"] / rf["steps"], "steps": rf["steps"], "batches_in_flight": fdepth,
                 "e2e": rf["e2e"], "converged_per_step": rf["conv_total"], "speedup_vs_parity_path": rf["value"] / value if value > 0 else None,
-                "quality": fq, "evals_per_step": int(fev.sum()), "roofline": roofline_of(rf, 32), "roofline_penalty": fpen}
+                "quality": fq, "evals_per_step": int(fev.sum()), "roofline": roofline_of(rf, 32), "roofline_penalty": fpen,
+                "note": None if rf["steps"] >= 3 * fdepth else
+                        "%d timed steps over %d lanes: the figure is dominated by filling and draining the pipeline; --steps %d or more measures "
+                        "the steady state" % (rf["steps"], fdepth, 3 * fdepth)}
         fo.close()
 
     # ---------------- CPU baseline on this box's host cores (rank 0, bounded sample) ----------------

@@ -5,7 +5,6 @@ The solve is chaotic with respect to last-bit differences (a 1e-15 input perturb
 vectors by ~1e-2; see DESIGN.md), so the CUDA path is built to be BIT-IDENTICAL to the oracle and these tests assert
 REL_TOL = 0 on everything that feeds a decision (cost, gradient, constraints, scales, iteration counts) and on the outputs.
 """
-import hashlib
 import os
 
 import numpy as np
@@ -119,15 +118,13 @@ def test_full_solve_matches_oracle_hill(gpu, hill_map):
 
 
 @pytest.mark.parametrize("name", ["hill", "desert", "volcano", "forest"])
-def test_full_solve_matches_golden_fixture(gpu, terrain, name):
+def test_full_solve_matches_golden_fixture(gpu, terrain, golden, name):
     """committed oracle outputs per terrain with the parameter sets of BASELINE configs 1-5 (tests/golden/make_golden.py,
     uneven_planner_b200/configs.py): hill; desert (== hill); volcano (max_sig 0.08 + config 4's max_kap 0.3, 64 samples per
     piece); forest (no scaling, rho_T 500, max_sig 0.001)"""
     from uneven_planner_b200 import configs, problems
     m = terrain(name)
-    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", f"{name}_oracle_golden.npz"))
-    if hashlib.sha256(m.cells.tobytes()).hexdigest() != str(gold["map_sha256"]):
-        pytest.skip(f"{name}.umap differs from the golden's")
+    gold = golden(name, m)
     pb = problems.generate(m, int(gold["B"]), seed=int(gold["seed"]), **configs.gen_kwargs(name))
     opt = gpu.BatchALMTrajOpt().init(configs.params_for(name)).set_environment(m)
     res, cxy, cyaw = opt.optimize(pb)
@@ -156,9 +153,9 @@ def test_cuda_matches_reference_build_directly(gpu, bumps_map):
     import ctypes as C
     import contextlib
     from uneven_planner_b200 import _lib, problems
-    from test_ref_pin import REF, _ref_solve
+    from test_ref_pin import NO_REF, REF, _ref_solve
     if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/libref.so not present (built where /root/reference exists; travels with the snapshot)")
+        pytest.skip(NO_REF % "libref.so")
     L = C.CDLL(REF)
     params = _lib.default_params()
     pb = problems.generate(bumps_map, 5, seed=21)

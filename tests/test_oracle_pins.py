@@ -275,14 +275,11 @@ def test_init_scaling_definition(bumps_map):
 
 # ---------------------------------------------------------------- (8) frozen outputs
 @pytest.mark.parametrize("name", ["hill", "desert", "volcano", "forest"])
-def test_oracle_matches_golden_fixture(terrain, name):
+def test_oracle_matches_golden_fixture(terrain, golden, name):
     """frozen oracle outputs per terrain / BASELINE config parameter set (tests/golden/make_golden.py)"""
-    import hashlib, os
     from uneven_planner_b200 import configs
     m = terrain(name)
-    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", f"{name}_oracle_golden.npz"))
-    if hashlib.sha256(m.cells.tobytes()).hexdigest() != str(gold["map_sha256"]):
-        pytest.skip(f"{name}.umap differs from the one the golden file was generated on")
+    gold = golden(name, m)
     pb = problems.generate(m, int(gold["B"]), seed=int(gold["seed"]), **configs.gen_kwargs(name))
     prm = po.params_from(configs.params_for(name))
     out = po.solve_batch(prm, po.OracleMap(m), pb, threads=4)

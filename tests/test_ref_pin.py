@@ -6,7 +6,12 @@ against oracle/shim (a minimal Eigen stand-in; Eigen and ROS are absent from thi
 (oracle/oracle.cpp) and require BIT-IDENTICAL outputs for MinJerkOpt<1|2>::generate / getTrajJerkCost / calJerkGradCT /
 calGradCTtoQT (SURVEY 8a rows a4-a6, a9, through BandedSystem a5) and for lbfgs_optimize + line_search_lewisoverton with the
 reference's local modifications (row a2, quirk Q8).  The shim fixes what the reference leaves to Eigen: dot()/norm() in the
-oracle's canonical 32-lane order, sum() in element order (oracle/shim/Eigen/Eigen header comment)."""
+oracle's canonical 32-lane order, sum() in element order (oracle/shim/Eigen/Eigen header comment).
+
+Every test here needs oracle/_ref/, which only `make -C oracle ref` builds from a checkout of the reference project; that project is
+not part of this repository, so on a checkout without that build each of them skips and says so.  Their reference outputs are not
+stored under tests/golden/ yet: recording them needs that build.  tests/golden/make_kino_golden.py is the pattern, and so far only
+KinoAstar's paths are recorded (tests/test_host_tools.py::test_kino_astar_reproduces_the_reference_golden_paths)."""
 import ctypes as C
 import os
 
@@ -15,6 +20,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = os.path.join(ROOT, "oracle", "_ref", "libref.so")
+NO_REF = ("oracle/_ref/%s not built: it is compiled from the reference project's sources (make -C oracle ref), which are not part of "
+          "this repository, and its outputs are not recorded under tests/golden/")
 dp = C.POINTER(C.c_double)
 
 
@@ -28,7 +35,7 @@ def ref(built):
         import subprocess
         subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "ref"], check=True)
     if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/libref.so not built (needs /root/reference; it travels to the GPU box prebuilt)")
+        pytest.skip(NO_REF % "libref.so")
     L = C.CDLL(REF)
     L.ref_minco.restype = C.c_int
     L.ref_minco.argtypes = [C.c_int, C.c_int, dp, dp, dp, dp, dp, dp, dp, dp, dp, dp, dp]
@@ -373,7 +380,7 @@ def reference_construct_map(cloud, size, iter_num=2, ellipsoid=(0.2, 0.1, 0.1)):
     preprocessed cloud: cells [X, Y, Yaw, 4] in double."""
     from uneven_planner_b200 import _lib
     if not os.path.exists(REFMAP):
-        pytest.skip("oracle/_ref/librefmap.so not built (needs the reference sources at build time)")
+        pytest.skip(NO_REF % "librefmap.so")
     R = C.CDLL(REFMAP)
     geom = _lib.map_geometry(size, size, 0.05, 0.1)
     X, Y, W = geom.voxel_num
@@ -448,7 +455,7 @@ REFKINO = os.path.join(ROOT, "oracle", "_ref", "librefkino.so")
 @pytest.fixture(scope="module")
 def refkino(ref):
     if not os.path.exists(REFKINO):
-        pytest.skip("oracle/_ref/librefkino.so not built")
+        pytest.skip(NO_REF % "librefkino.so")
     L = C.CDLL(REFKINO)
     u8 = C.POINTER(C.c_uint8)
     L.ref_kino_plan.argtypes = [dp, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, dp, dp, dp, dp, C.c_int, u8, u8]

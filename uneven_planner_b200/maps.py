@@ -128,6 +128,17 @@ def get_terrain(name, build_if_missing=True):
     return None
 
 
+# Seeded synthetic stand-ins of the reference's terrains, for tests where maps_built/<name>.umap cannot be had (the reference's
+# point clouds are not part of this repository).  hill's stand-in is the terrain bench.py falls back to.
+STANDIN_SEED = {"hill": 0, "desert": 1, "volcano": 2, "forest": 4}
+
+
+def terrain_or_standin(name):
+    """The reference terrain `name` when its .umap exists (or can be built), else its seeded synthetic stand-in.  A stand-in is
+    NOT the reference terrain: results on it compare implementations with each other, not with the reference's maps."""
+    return get_terrain(name) or synthetic_terrain("bumps", seed=STANDIN_SEED[name])
+
+
 def synthetic_terrain(kind="bumps", seed=0, size=(200, 200, 64)):
     """Analytic terrain z = h(x,y) turned into the same grid the builder produces (normal of the surface
     at the 0.12 m forward-shifted footprint centre, sigma from curvature).  Used by tests and as a clearly
