@@ -271,6 +271,27 @@ int ualm_front_end_batch(const ualm_astar_map_t *map, const ualm_astar_params_t 
                          const double *starts, const double *goals, int nthreads, int32_t *N, int32_t *M, double *bnd, double *total_time,
                          double *inner_xy, long long cap_xy, double *inner_yaw, long long cap_yaw, int32_t *packed, int32_t *n_expanded);
 
+/* The same search on the host with include/ualm_detmath.h's sin / cos / tan / atan2 / acos instead of the C library's: bit for bit
+ * what ualm_front_end_batch_device computes for one pair.  For tests; it differs from ualm_kino_astar_plan only in the trigonometry. */
+int ualm_kino_astar_plan_det(const ualm_astar_map_t *map, const ualm_astar_params_t *p, const double start[3], const double goal[3],
+                             double *path_xyyaw, int max_pts, int *n_expanded);
+
+/* ---- the front-end on the GPU (csrc/ualm_front_end.cu): one warp per KinoAstar search ----
+ * ualm_set_front_end_map: uploads the occupancy grids and the cell grid (double when map->cells64 is set, float otherwise, as the host
+ * search reads it) to the context's device.
+ * ualm_front_end_batch_device: ualm_front_end_batch's outputs for B pairs, searched on the device with ualm_kino_astar_plan_det's
+ * arithmetic (bit-identical to it; the trigonometry makes it differ from ualm_front_end_batch in the last bits), resampled on the host by
+ * ualm_resample_path.  A polyline longer than ualm_front_end_path_cap points cannot pass the optimizer's limits: it is left out
+ * (packed = -1) and returned empty.  Optional: path_xyyaw (room for cap_path points) + path_off[B + 1], the raw polylines back to back;
+ * search_ms, the CUDA-event time of the search kernel.  Poses must be finite with |yaw| <= 1e4 and the A* parameters finite. */
+int ualm_set_front_end_map(ualm_ctx_t *ctx, const ualm_astar_map_t *map);
+int ualm_front_end_batch_device(ualm_ctx_t *ctx, const ualm_astar_params_t *ap, const ualm_resample_params_t *rp, int B, const double *starts,
+                                const double *goals, int32_t *N, int32_t *M, double *bnd, double *total_time, double *inner_xy, long long cap_xy,
+                                double *inner_yaw, long long cap_yaw, int32_t *packed, int32_t *n_expanded, double *path_xyyaw, long long cap_path,
+                                int64_t *path_off, float *search_ms);
+/* the most points one device search returns for these parameters: every polyline the resampler can accept within N <= 64, M <= 128 fits */
+int ualm_front_end_path_cap(const ualm_astar_params_t *ap, const ualm_resample_params_t *rp);
+
 #ifdef __cplusplus
 }
 #endif

@@ -114,4 +114,10 @@ UALM_HD double ualm_atan2(double y, double x)
     return y > 0.0 ? r : -r;
 }
 
+/* tan and acos for the front-end (turning radius, motion primitives, the Dubins words RLR / LRL), from the kernels above with
+ * one more IEEE operation: tan = sin / cos of one reduction, acos(x) = atan2(sqrt((1 - x)(1 + x)), x), which keeps its accuracy as
+ * |x| -> 1 where 1 - x*x would cancel.  NaN outside [-1, 1] like libm. */
+UALM_HD double ualm_tan(double x) { double s, c; ualm_sincos(x, &s, &c); return s / c; }
+UALM_HD double ualm_acos(double x) { return ualm_atan2(sqrt((1.0 - x) * (1.0 + x)), x); }
+
 #endif

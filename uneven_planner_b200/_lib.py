@@ -74,6 +74,7 @@ def lib():
     L.ualm_astar_default_params.argtypes = [C.POINTER(AstarParams)]
     L.ualm_astar_default_params.restype = None
     L.ualm_kino_astar_plan.argtypes = [C.POINTER(AstarMap), C.POINTER(AstarParams), dp, dp, dp, C.c_int, C.POINTER(C.c_int)]
+    L.ualm_kino_astar_plan_det.argtypes = [C.POINTER(AstarMap), C.POINTER(AstarParams), dp, dp, dp, C.c_int, C.POINTER(C.c_int)]
     L.ualm_front_end_batch.argtypes = [C.POINTER(AstarMap), C.POINTER(AstarParams), C.POINTER(ResampleParams), C.c_int, dp, dp, C.c_int, ip, ip, dp, dp, dp,
                                        C.c_longlong, dp, C.c_longlong, ip, ip]
     L.ualm_resample_path.argtypes = [dp, C.c_int, C.c_double, C.c_double, C.c_double, C.c_double, C.c_double, dp, dp,
@@ -120,8 +121,13 @@ def lib():
         L.ualm_mark_end.argtypes = [vp, C.POINTER(C.c_float)]
         L.ualm_solve_batch_multi.argtypes = [C.POINTER(vp), C.c_int, C.c_int, ip, ip, dp, dp, dp, dp, C.POINTER(Result), dp, dp]
         L.ualm_pack_records_device_async.argtypes = [vp, vp, C.c_int]
+        L.ualm_set_front_end_map.argtypes = [vp, C.POINTER(AstarMap)]
+        L.ualm_front_end_batch_device.argtypes = [vp, C.POINTER(AstarParams), C.POINTER(ResampleParams), C.c_int, dp, dp, ip, ip, dp, dp, dp, C.c_longlong, dp,
+                                                  C.c_longlong, ip, ip, dp, C.c_longlong, C.POINTER(C.c_int64), C.POINTER(C.c_float)]
+        L.ualm_front_end_path_cap.argtypes = [C.POINTER(AstarParams), C.POINTER(ResampleParams)]
         for name in ("ualm_reset_stream", "ualm_set_map_f64", "ualm_max_lanes", "ualm_select_lane", "ualm_submit_batch", "ualm_wait_batch",
-                     "ualm_mark_begin", "ualm_mark_end", "ualm_solve_batch_multi", "ualm_pack_records_device_async"):
+                     "ualm_mark_begin", "ualm_mark_end", "ualm_solve_batch_multi", "ualm_pack_records_device_async", "ualm_set_front_end_map",
+                     "ualm_front_end_batch_device", "ualm_front_end_path_cap"):
             getattr(L, name).restype = C.c_int
         for name in ("ualm_create", "ualm_destroy", "ualm_set_params", "ualm_set_map", "ualm_solve_batch",
                      "ualm_upload", "ualm_solve_resident", "ualm_sync", "ualm_download", "ualm_last_solve_ms",

@@ -15,10 +15,11 @@ CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libualm.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-CU_SOURCES = ["ualm_api.cu"]          # parity path + C ABI: -fmad=false (bit-identical to the CPU oracle)
+CU_SOURCES = ["ualm_api.cu", "ualm_front_end.cu"]   # parity path, device front-end + C ABI: -fmad=false (bit-identical to the host)
 CU_SOURCES_FMA = ["ualm_tp.cu"]       # throughput path (precision 32 / 65): FMA contraction on, CUDA libm
 CXX_SOURCES = ["host_tools.cpp", "kino_astar.cpp"]
-HEADERS = ["ualm_kernels.cuh", "map_cell.h", "map_prep.h", "../../include/ualm_detmath.h", "ualm_tp_kernels.cuh", "ualm_tp_samples.cuh", "ualm_tp_host.h", "dubins.h"]
+HEADERS = ["ualm_kernels.cuh", "map_cell.h", "map_prep.h", "../../include/ualm_detmath.h", "ualm_tp_kernels.cuh", "ualm_tp_samples.cuh", "ualm_tp_host.h", "dubins.h", "kino_search.h",
+           "ualm_front_end.h"]
 
 
 

@@ -2,295 +2,83 @@
 // (front_end/src/kino_astar.cpp:67-236; helpers front_end/include/front_end/kino_astar.h:177-291) over the UnevenMap occupancy grids,
 // and the batch form that turns (start, goal) pairs into the optimizer's inputs:
 //     KinoAstar::plan -> PlanManager's resampler (ualm_resample_path, plan_manager.cpp:62-122) -> ualm_solve_batch / ualm_submit_batch.
-// The search is sequential by nature (one priority queue); a batch runs one search per host thread.
-//
-// Behaviour kept from the reference, because every one of these decides which path comes out:
-//   * hybrid-state grid: cell = (x, y) of the map and a yaw bin of kino_astar/yaw_resolution (NOT the map's) -- kino_astar.h:190-194;
-//   * 3 speeds x 5 steering angles per expansion, built by the same floating-point loops (kino_astar.cpp:128-136);
-//   * a node whose cost improves while OPEN is rewritten in place and NOT re-sorted in the queue (kino_astar.cpp:213-224): the queue is
-//     std::priority_queue over node pointers, exactly as there, so equal-f ties and stale orderings resolve the same way;
-//   * the goal test is "within oneshot_range and the Dubins one-shot is collision free", tried on the node at the top of the queue
-//     before it is popped (kino_astar.cpp:107-121); the result is start .. node, then the one-shot samples (kino_astar.h:268-291);
-//   * the node pool holds X * Y nodes (kino_astar.h:177-185); running out ends the search without a path.
-// Pinned bit for bit against kino_astar.cpp compiled unmodified (tests/test_ref_pin.py::test_kino_astar_*), with csrc/dubins.h standing
-// in for OMPL on both sides.
-#include <cmath>
+// The search itself is csrc/kino_search.h (shared with the device front-end, csrc/ualm_front_end.cu); here it runs with the C library's
+// trigonometry (TrigLibm), one search per host thread.  Pinned bit for bit against kino_astar.cpp compiled unmodified
+// (tests/test_ref_pin.py::test_kino_astar_*), with csrc/dubins.h standing in for OMPL on both sides.
+#include <algorithm>
+#include <atomic>
 #include <cstdint>
 #include <cstring>
-#include <queue>
 #include <thread>
-#include <atomic>
-#include <unordered_map>
 #include <vector>
 
-#include "dubins.h"
+#include "kino_search.h"
 #include "ualm.h"
+#include "ualm_front_end.h"
 
 namespace {
 
-struct MapView {
-    const ualm_map_geom_t *g;
-    const float *cells;
-    const double *cells64;
-    const uint8_t *occ3, *occ2;
-    double xy_inv, yaw_inv;
+using ualm_kino::MapView;
 
-    // uneven_map.h:411-417
-    void posToIndex(const double p[3], int id[3]) const
-    {
-        id[0] = (int)std::floor((p[0] - g->origin[0]) * xy_inv);
-        id[1] = (int)std::floor((p[1] - g->origin[1]) * xy_inv);
-        id[2] = (int)std::floor((p[2] - g->origin[2]) * yaw_inv);
-    }
-    // uneven_map.h:437-454
-    bool inMap(const double p[3]) const
-    {
-        for (int k = 0; k < 3; k++) if (p[k] < g->origin[k] + 1e-4) return false;
-        for (int k = 0; k < 3; k++) if (p[k] > g->max_boundary[k] - 1e-4) return false;
-        return true;
-    }
-    // uneven_map.h:456-471
-    bool inMapIdx(const int id[3]) const
-    {
-        if (id[0] < 0 || id[1] < 0 || id[2] < 0) return false;
-        return !(id[0] > g->voxel_num[0] - 1 || id[1] > g->voxel_num[1] - 1 || id[2] > g->voxel_num[2] - 1);
-    }
-    size_t addr(int x, int y, int w) const { return (size_t)x * g->voxel_num[1] * g->voxel_num[2] + (size_t)y * g->voxel_num[2] + w; }
-    // uneven_map.h:473-488
-    int occupancy(const double p[3]) const
-    {
-        int id[3];
-        posToIndex(p, id);
-        if (!inMapIdx(id)) return -1;
-        return (int)occ3[addr(id[0], id[1], id[2])];
-    }
-    // uneven_map.h:490-500
-    int occupancyXY(const double p[3]) const
-    {
-        int id[3];
-        posToIndex(p, id);
-        if (!inMapIdx(id)) return -1;
-        return (int)occ2[(size_t)id[0] * g->voxel_num[1] + id[1]];
-    }
-    double sigma_at(int x, int y, int w) const
-    {
-        const size_t a = addr(x, y, w);
-        return cells64 ? cells64[4 * a + 1] : (double)cells[4 * a + 1];
-    }
-    // UnevenMap::getTerrainSig = the sigma component of getTerrain's trilinear blend (uneven_map.h:154-201, 389-396)
-    double terrainSig(const double pos[3]) const
-    {
-        if (!inMap(pos)) return 0.0;
-        double pm[3] = {pos[0] - 0.5 * g->xy_resolution, pos[1] - 0.5 * g->xy_resolution, pos[2] - 0.5 * g->yaw_resolution};
-        while (pm[2] < -M_PI) pm[2] += 2 * M_PI;       // normSO2, uneven_map.cpp:64-71
-        while (pm[2] > M_PI) pm[2] -= 2 * M_PI;
-        int idx[3];
-        posToIndex(pm, idx);
-        const double ip[3] = {(idx[0] + 0.5) * g->xy_resolution + g->origin[0], (idx[1] + 0.5) * g->xy_resolution + g->origin[1],
-                              (idx[2] + 0.5) * g->yaw_resolution + g->origin[2]};
-        double diff[3] = {(pos[0] - ip[0]) * xy_inv, (pos[1] - ip[1]) * xy_inv, 0.0};
-        diff[2] = std::atan2(std::sin(pos[2] - ip[2]), std::cos(pos[2] - ip[2])) * yaw_inv;
-        double v[2][2][2];
-        for (int x = 0; x < 2; x++)
-            for (int y = 0; y < 2; y++)
-                for (int w = 0; w < 2; w++) {
-                    int c[3] = {idx[0] + x, idx[1] + y, idx[2] + w};
-                    c[0] = std::max(std::min(c[0], g->voxel_num[0] - 1), 0);       // boundIndex, uneven_map.h:398-409
-                    c[1] = std::max(std::min(c[1], g->voxel_num[1] - 1), 0);
-                    while (c[2] > g->voxel_num[2] - 1) c[2] -= g->voxel_num[2];
-                    while (c[2] < 0) c[2] += g->voxel_num[2];
-                    v[x][y][w] = sigma_at(c[0], c[1], c[2]);
-                }
-        const double v00 = v[0][0][0] * (1 - diff[0]) + v[1][0][0] * diff[0];
-        const double v01 = v[0][0][1] * (1 - diff[0]) + v[1][0][1] * diff[0];
-        const double v10 = v[0][1][0] * (1 - diff[0]) + v[1][1][0] * diff[0];
-        const double v11 = v[0][1][1] * (1 - diff[0]) + v[1][1][1] * diff[0];
-        const double v0 = v00 * (1 - diff[1]) + v10 * diff[1];
-        const double v1 = v01 * (1 - diff[1]) + v11 * diff[1];
-        return v0 * (1 - diff[2]) + v1 * diff[2];
-    }
-};
-
-enum : char { ST_CLOSE = 'a', ST_OPEN = 'b', ST_NOT_EXPAND = 'c' };
-struct Node {
-    int index[3];
-    double state[3];
-    double input[2];
-    double g_score, f_score;
-    char node_state = ST_NOT_EXPAND;
-    Node *parent = nullptr;
-};
-struct ByF { bool operator()(const Node *a, const Node *b) const { return a->f_score > b->f_score; } };
-struct Key { int x, y, w; bool operator==(const Key &o) const { return x == o.x && y == o.y && w == o.w; } };
-struct KeyHash { size_t operator()(const Key &k) const { return ((size_t)(uint32_t)k.x * 73856093u) ^ ((size_t)(uint32_t)k.y * 19349663u) ^ ((size_t)(uint32_t)k.w * 83492791u); } };
-
-double norm_angle(double a)        // kino_astar.h:196-207
+bool params_ok(const ualm_astar_params_t *p)
 {
-    while (a > M_PI) a -= 6.283185307179586;
-    while (a < -M_PI) a += 6.283185307179586;
-    return a;
-}
-// kino_astar.h:220-244
-void state_transit(const ualm_astar_params_t &p, const double s0[3], double s1[3], const double in[2], double T)
-{
-    const double v = in[0], delta = in[1];
-    const double s = v * T;
-    const double y = s * std::tan(delta) / p.wheel_base;
-    if (std::fabs(delta) > 1e-4) {
-        const double r = s / y;
-        s1[0] = s0[0] + r * (std::sin(s0[2] + y) - std::sin(s0[2]));
-        s1[1] = s0[1] - r * (std::cos(s0[2] + y) - std::cos(s0[2]));
-        s1[2] = s0[2] + y;
-        s1[2] = norm_angle(s1[2]);
-    } else {
-        s1[0] = s0[0] + s * std::cos(s0[2]);
-        s1[1] = s0[1] + s * std::sin(s0[2]);
-        s1[2] = s0[2];
-    }
+    return p && p->yaw_resolution > 0 && p->max_vel > 0 && p->max_steer > 0 && p->collision_interval > 0 && p->time_interval > 0 && p->wheel_base > 0;
 }
 
-struct Planner {
-    const MapView &map;
-    const ualm_astar_params_t &p;
-    std::vector<Node> pool;
-    double yaw_inv;
-    const double tie_breaker = 1.0 + 1.0 / 10000;
+// one host thread's search state: the node pool (X * Y nodes), OPEN, the expanded-node table, the inputs and the one-shot's samples
+template <class T> struct Planner {
+    ualm_kino::Search<T> s;
+    std::vector<ualm_kino::Node> pool;
+    std::vector<int> heap, table;
+    std::vector<double> inputs, shot;
+    int nin, shot_cap;
 
-    Planner(const MapView &m, const ualm_astar_params_t &pp) : map(m), p(pp), pool((size_t)m.g->voxel_num[0] * m.g->voxel_num[1]), yaw_inv(1.0 / pp.yaw_resolution) {}
-
-    void state_to_index(const double s[3], int id[3]) const    // kino_astar.h:190-194
+    Planner(const MapView &m, const ualm_astar_params_t &p) : pool((size_t)m.g.voxel_num[0] * m.g.voxel_num[1]), heap(pool.size()),
+                                                            table(ualm_kino::table_capacity((long long)pool.size()))
     {
-        map.posToIndex(s, id);
-        id[2] = (int)std::floor((norm_angle(s[2]) + M_PI) * yaw_inv);
+        s.map = m; s.p = p; s.yaw_inv = 1.0 / p.yaw_resolution;
+        s.rho = p.wheel_base / T::tan(p.max_steer);
+        s.pool = pool.data(); s.pool_size = (int)pool.size();
+        s.open.h = heap.data(); s.open.n = 0;
+        s.closed.slot = table.data(); s.closed.mask = (unsigned)table.size() - 1;
+        nin = ualm_kino::build_inputs(p, nullptr, 0);
+        inputs.resize(2 * (size_t)nin);
+        ualm_kino::build_inputs(p, inputs.data(), nin);
+        shot_cap = std::max(ualm_kino::shot_capacity(p, s.rho), 1);
+        shot.resize(3 * (size_t)shot_cap);
     }
-    double heu(const double a[3], const double b[3]) const     // kino_astar.h:215-218
-    {
-        const double dx = a[0] - b[0], dy = a[1] - b[1];
-        return tie_breaker * std::sqrt(dx * dx + dy * dy);
-    }
-    // kino_astar.h:246-266: the Dubins curve sampled every collision_interval, empty if any sample is occupied
-    void shot(const double s1[3], const double s2[3], std::vector<double> &out) const
-    {
-        out.clear();
-        const double rho = p.wheel_base / std::tan(p.max_steer);
-        const ualm_dubins::Path path = ualm_dubins::shortest(s1, s2, rho);
-        const double len = rho * path.length();
-        for (double l = 0.0; l <= len; l += p.collision_interval) {
-            double q[3];
-            ualm_dubins::interpolate(s1, path, rho, l / len, q);
-            out.insert(out.end(), q, q + 3);
-        }
-        for (size_t i = 0; i < out.size() / 3; i++)
-            if (map.occupancyXY(&out[3 * i]) == 1) { out.clear(); break; }
-    }
-
-    // KinoAstar::plan (kino_astar.cpp:67-236).  path: (x, y, yaw) triples; expanded: nodes closed
-    void plan(const double start[3], const double goal[3], std::vector<double> &path, int *expanded)
+    // path: (x, y, yaw) triples, empty without a path; expanded: nodes closed.  UALM_OK, or UALM_ELIMIT if the one-shot had more
+    // samples than shot_capacity allows for (it cannot)
+    int plan(const double start[3], const double goal[3], std::vector<double> &path, int *expanded)
     {
         path.clear();
-        if (expanded) *expanded = 0;
-        int use_node_num = 0, iter_num = 0;
-        std::priority_queue<Node *, std::vector<Node *>, ByF> open_set;
-        std::unordered_map<Key, Node *, KeyHash> expanded_nodes;
-        if (map.occupancy(start) == 1) return;
-        if (map.occupancyXY(goal) == 1) return;
-        Node *cur = &pool[0];
-        cur->parent = nullptr;
-        cur->state[0] = start[0]; cur->state[1] = start[1]; cur->state[2] = norm_angle(start[2]);
-        state_to_index(cur->state, cur->index);
-        cur->g_score = 0.0;
-        cur->input[0] = 0.0; cur->input[1] = 0.0;
-        cur->f_score = p.lambda_heu * heu(cur->state, goal);
-        cur->node_state = ST_OPEN;
-        open_set.push(cur);
-        use_node_num += 1;
-        expanded_nodes.insert({Key{cur->index[0], cur->index[1], cur->index[2]}, cur});
-        std::vector<double> shot_path;
-        std::vector<double> inputs;
-        while (!open_set.empty()) {
-            cur = open_set.top();
-            const double ex = cur->state[0] - goal[0], ey = cur->state[1] - goal[1];
-            if (std::sqrt(ex * ex + ey * ey) < p.oneshot_range) {
-                shot(cur->state, goal, shot_path);
-                if (!shot_path.empty()) {
-                    // retrievePath (kino_astar.h:268-291): the chain back to the start, reversed, then the one-shot samples
-                    std::vector<const Node *> chain;
-                    for (const Node *n = cur; n; n = n->parent) chain.push_back(n);
-                    for (size_t k = chain.size(); k-- > 0;) path.insert(path.end(), chain[k]->state, chain[k]->state + 3);
-                    path.insert(path.end(), shot_path.begin(), shot_path.end());
-                    if (expanded) *expanded = iter_num;
-                    return;
-                }
-            }
-            open_set.pop();
-            cur->node_state = ST_CLOSE;
-            iter_num += 1;
-            const double cur_state[3] = {cur->state[0], cur->state[1], cur->state[2]};
-            inputs.clear();
-            for (double v = 0; v <= p.max_vel + 1e-3; v += 0.5 * p.max_vel)
-                for (double steer = -p.max_steer; steer <= p.max_steer + 1e-3; steer += 0.5 * p.max_steer) { inputs.push_back(v); inputs.push_back(steer); }
-            for (size_t i = 0; i < inputs.size() / 2; i++) {
-                const double input[2] = {inputs[2 * i], inputs[2 * i + 1]};
-                double pro_state[3];
-                state_transit(p, cur_state, pro_state, input, p.time_interval);
-                if (!map.inMap(pro_state)) continue;
-                int pro_id[3];
-                state_to_index(pro_state, pro_id);
-                auto it = expanded_nodes.find(Key{pro_id[0], pro_id[1], pro_id[2]});
-                Node *pro = it == expanded_nodes.end() ? nullptr : it->second;
-                if (pro && pro->node_state == ST_CLOSE) continue;
-                int occ = 0;
-                const double arc = input[0] * p.time_interval;
-                const double temp_ct = p.collision_interval / arc * p.time_interval;
-                for (double t = temp_ct; t <= p.time_interval + 1e-3; t += temp_ct) {
-                    double xt[3];
-                    state_transit(p, cur_state, xt, input, t);
-                    occ = map.occupancyXY(xt);
-                    if (occ == 1) break;
-                }
-                if (occ == 1) continue;
-                double g = 0.0;
-                g += p.weight_r2 * arc;
-                g += p.weight_so2 * std::fabs(input[1]) * arc;
-                g += p.weight_v_change * std::fabs(input[0] - cur->input[0]);
-                g += p.weight_delta_change * std::fabs(input[1] - cur->input[1]);
-                g += p.weight_sigma * map.terrainSig(pro_state);
-                g += cur->g_score;
-                const double f = g + p.lambda_heu * heu(pro_state, goal);
-                if (!pro) {
-                    pro = &pool[use_node_num];
-                    std::memcpy(pro->index, pro_id, sizeof(pro_id));
-                    std::memcpy(pro->state, pro_state, sizeof(pro_state));
-                    pro->f_score = f; pro->g_score = g;
-                    pro->input[0] = input[0]; pro->input[1] = input[1];
-                    pro->parent = cur;
-                    pro->node_state = ST_OPEN;
-                    open_set.push(pro);
-                    expanded_nodes.insert({Key{pro_id[0], pro_id[1], pro_id[2]}, pro});
-                    use_node_num++;
-                    if (use_node_num == (int)pool.size()) { if (expanded) *expanded = iter_num; return; }      // "run out of memory."
-                } else if (pro->node_state == ST_OPEN) {
-                    if (g < pro->g_score) {
-                        std::memcpy(pro->index, pro_id, sizeof(pro_id));
-                        std::memcpy(pro->state, pro_state, sizeof(pro_state));
-                        pro->f_score = f; pro->g_score = g;
-                        pro->input[0] = input[0]; pro->input[1] = input[1];
-                        pro->parent = cur;
-                    }
-                }
-            }
+        std::fill(table.begin(), table.end(), -1);
+        int node = -1, nshot = 0;
+        const int st = s.plan(start, goal, inputs.data(), nin, shot.data(), shot_cap, &node, &nshot);
+        if (expanded) *expanded = s.iter_num;
+        if (st == ualm_kino::KS_SHOT_OVERFLOW) return UALM_ELIMIT;
+        if (st == ualm_kino::KS_FOUND) {
+            const int chain = s.chain_length(node);
+            path.resize(3 * (size_t)(chain + nshot));
+            s.retrieve(node, chain, shot.data(), nshot, path.data());
         }
-        if (expanded) *expanded = iter_num;
+        return UALM_OK;
     }
-    void reset_pool(int used) { for (int i = 0; i < used && i < (int)pool.size(); i++) { pool[i].parent = nullptr; pool[i].node_state = ST_NOT_EXPAND; } }
 };
 
-bool view_of(const ualm_astar_map_t *m, MapView &v)
+template <class T> int plan_one(const ualm_astar_map_t *map, const ualm_astar_params_t *p, const double start[3], const double goal[3], double *path_xyyaw,
+                                int max_pts, int *n_expanded)
 {
-    if (!m || !m->geom || (!m->cells && !m->cells64) || !m->occ3 || !m->occ2) return false;
-    v.g = m->geom; v.cells = m->cells; v.cells64 = m->cells64; v.occ3 = m->occ3; v.occ2 = m->occ2;
-    v.xy_inv = 1.0 / m->geom->xy_resolution; v.yaw_inv = 1.0 / m->geom->yaw_resolution;
-    return true;
+    MapView v;
+    if (!ualm_kino::view_of(map, v) || !params_ok(p) || !start || !goal || !path_xyyaw || max_pts < 0) return UALM_EINVAL;
+    Planner<T> pl(v, *p);
+    std::vector<double> path;
+    const int rc = pl.plan(start, goal, path, n_expanded);
+    if (rc != UALM_OK) return rc;
+    const int n = (int)(path.size() / 3);
+    if (n > max_pts) return UALM_ELIMIT;
+    std::memcpy(path_xyyaw, path.data(), sizeof(double) * path.size());
+    return n;
 }
 
 } // namespace
@@ -306,17 +94,14 @@ extern "C" void ualm_astar_default_params(ualm_astar_params_t *p)
 extern "C" int ualm_kino_astar_plan(const ualm_astar_map_t *map, const ualm_astar_params_t *p, const double start[3], const double goal[3], double *path_xyyaw,
                                     int max_pts, int *n_expanded)
 {
-    MapView v;
-    if (!view_of(map, v) || !p || !start || !goal || !path_xyyaw || max_pts < 0) return UALM_EINVAL;
-    if (!(p->yaw_resolution > 0) || !(p->max_vel > 0) || !(p->max_steer > 0) || !(p->collision_interval > 0) || !(p->time_interval > 0) || !(p->wheel_base > 0))
-        return UALM_EINVAL;
-    Planner pl(v, *p);
-    std::vector<double> path;
-    pl.plan(start, goal, path, n_expanded);
-    const int n = (int)(path.size() / 3);
-    if (n > max_pts) return UALM_ELIMIT;
-    std::memcpy(path_xyyaw, path.data(), sizeof(double) * path.size());
-    return n;
+    return plan_one<TrigLibm>(map, p, start, goal, path_xyyaw, max_pts, n_expanded);
+}
+
+// the same search with include/ualm_detmath.h's trigonometry: the host twin of ualm_front_end_batch_device, for tests
+extern "C" int ualm_kino_astar_plan_det(const ualm_astar_map_t *map, const ualm_astar_params_t *p, const double start[3], const double goal[3],
+                                        double *path_xyyaw, int max_pts, int *n_expanded)
+{
+    return plan_one<TrigDet>(map, p, start, goal, path_xyyaw, max_pts, n_expanded);
 }
 
 // the one-shot curve alone (kino_astar.h:246-258 without the occupancy test): samples every `interval` metres of the shortest Dubins
@@ -324,13 +109,13 @@ extern "C" int ualm_kino_astar_plan(const ualm_astar_map_t *map, const ualm_asta
 extern "C" int ualm_dubins_shot(const double start[3], const double goal[3], double radius, double interval, double *path_xyyaw, int max_pts, double *length)
 {
     if (!start || !goal || !path_xyyaw || !(radius > 0) || !(interval > 0) || max_pts < 1) return UALM_EINVAL;
-    const ualm_dubins::Path path = ualm_dubins::shortest(start, goal, radius);
+    const ualm_dubins::Path path = ualm_dubins::shortest<TrigLibm>(start, goal, radius);
     const double len = radius * path.length();
     if (length) *length = len;
     int n = 0;
     for (double l = 0.0; l <= len; l += interval) {
         if (n >= max_pts) return UALM_ELIMIT;
-        ualm_dubins::interpolate(start, path, radius, l / len, path_xyyaw + 3 * n);
+        ualm_dubins::interpolate<TrigLibm>(start, path, radius, l / len, path_xyyaw + 3 * n);
         n++;
     }
     return n;
@@ -344,37 +129,48 @@ extern "C" int ualm_front_end_batch(const ualm_astar_map_t *map, const ualm_asta
                                     long long cap_xy, double *inner_yaw, long long cap_yaw, int32_t *packed, int32_t *n_expanded)
 {
     MapView v;
-    if (!view_of(map, v) || !ap || !rp || B < 0 || (B > 0 && (!starts || !goals || !N || !M || !bnd || !total_time || !inner_xy || !inner_yaw || !packed))) return UALM_EINVAL;
-    struct One { int ok = 0; int32_t N = 0, M = 0; double T = 0; double bnd[18]; std::vector<double> ixy, iyaw; int expanded = 0; };
-    std::vector<One> res(B);
+    if (!ualm_kino::view_of(map, v) || !ap || !rp || B < 0 || (B > 0 && (!starts || !goals || !N || !M || !bnd || !total_time || !inner_xy || !inner_yaw || !packed))) return UALM_EINVAL;
+    std::vector<ualm_fe::Resampled> res(B);
+    std::vector<int> expanded(B, 0), rcs(B, UALM_OK);
     std::atomic<int> next(0);
     if (nthreads <= 0) nthreads = (int)std::max(1u, std::thread::hardware_concurrency());
     nthreads = std::min(nthreads, std::max(B, 1));
     auto worker = [&]() {
-        Planner pl(v, *ap);
+        Planner<TrigLibm> pl(v, *ap);
         std::vector<double> path;
         for (;;) {
             const int b = next.fetch_add(1);
             if (b >= B) break;
-            One &o = res[b];
-            pl.plan(starts + 3 * b, goals + 3 * b, path, &o.expanded);
-            pl.reset_pool((int)pl.pool.size());
-            const int npts = (int)(path.size() / 3);
-            if (npts < 2) continue;
-            o.ixy.assign(2 * 64, 0.0); o.iyaw.assign(128, 0.0);
-            const int rc = ualm_resample_path(path.data(), npts, rp->piece_len, rp->yaw_piece_times, rp->mean_vel, rp->init_time_times, rp->init_sig_vel, o.bnd,
-                                              o.ixy.data(), 63, o.iyaw.data(), 127, &o.N, &o.M, &o.T);      // N <= 64, M <= 128: the optimizer's limits
-            o.ok = rc == UALM_OK;
+            rcs[b] = pl.plan(starts + 3 * b, goals + 3 * b, path, &expanded[b]);
+            ualm_fe::resample(path.data(), (int)(path.size() / 3), rp, res[b]);
         }
     };
     std::vector<std::thread> th;
     for (int t = 0; t < nthreads; t++) th.emplace_back(worker);
     for (auto &t : th) t.join();
+    for (int b = 0; b < B; b++)
+        if (rcs[b] != UALM_OK) return rcs[b];
+    if (n_expanded) std::copy(expanded.begin(), expanded.end(), n_expanded);
+    return ualm_fe::pack(res, N, M, bnd, total_time, inner_xy, cap_xy, inner_yaw, cap_yaw, packed);
+}
+
+void ualm_fe::resample(const double *path, int npts, const ualm_resample_params_t *rp, Resampled &o)
+{
+    o.ok = 0;
+    if (npts < 2) return;
+    o.ixy.assign(2 * 64, 0.0); o.iyaw.assign(128, 0.0);
+    const int rc = ualm_resample_path(path, npts, rp->piece_len, rp->yaw_piece_times, rp->mean_vel, rp->init_time_times, rp->init_sig_vel, o.bnd,
+                                      o.ixy.data(), 63, o.iyaw.data(), 127, &o.N, &o.M, &o.T);      // N <= 64, M <= 128: the optimizer's limits
+    o.ok = rc == UALM_OK;
+}
+
+int ualm_fe::pack(const std::vector<Resampled> &res, int32_t *N, int32_t *M, double *bnd, double *total_time, double *inner_xy, long long cap_xy,
+                  double *inner_yaw, long long cap_yaw, int32_t *packed)
+{
     int k = 0;
     long long oxy = 0, oyaw = 0;
-    for (int b = 0; b < B; b++) {
-        const One &o = res[b];
-        if (n_expanded) n_expanded[b] = o.expanded;
+    for (size_t b = 0; b < res.size(); b++) {
+        const Resampled &o = res[b];
         packed[b] = -1;
         if (!o.ok) continue;
         if (oxy + 2LL * (o.N - 1) > cap_xy || oyaw + (o.M - 1) > cap_yaw) return UALM_ELIMIT;

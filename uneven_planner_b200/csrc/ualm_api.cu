@@ -5,6 +5,7 @@
 #include "ualm_kernels.cuh"
 #include "map_prep.h"
 #include "ualm_tp_host.h"
+#include "ualm_front_end.h"
 
 #include <algorithm>
 #include <cstdio>
@@ -111,6 +112,7 @@ struct ualm_ctx {
     // pipeline timing (ualm_mark_begin / ualm_mark_end): events on the lanes' own streams, joined on `join`
     cudaStream_t join = nullptr;
     cudaEvent_t evA = nullptr, evB = nullptr;
+    ualm_fe::FrontEnd *fe = nullptr;     // the device front-end's map and workspaces (ualm_set_front_end_map)
 };
 
 static int lane_make(ualm_ctx *c, Lane &l)
@@ -179,6 +181,7 @@ extern "C" int ualm_destroy(ualm_ctx_t *c)
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     if (c->tp) { ualm_tp::tp_destroy(c->tp); c->tp = nullptr; }
+    ualm_fe::release(c->fe); c->fe = nullptr;
     c->cells.release(); c->cells64.release();
     for (auto &l : c->lanes) l.release();
     if (c->join) cudaStreamDestroy(c->join);
@@ -1058,4 +1061,33 @@ extern "C" int ualm_map_build_device(ualm_ctx_t *c, const float *pin, int64_t np
     CK(cudaStreamSynchronize(c->b->stream));
     if (kernel_ms) CK(cudaEventElapsedTime(kernel_ms, sc.e0, sc.e1));
     return UALM_OK;
+}
+
+// ---- the front-end on the device (csrc/ualm_front_end.cu) ----
+extern "C" int ualm_set_front_end_map(ualm_ctx_t *c, const ualm_astar_map_t *m)
+{
+    if (!c || !m) return fail(UALM_EINVAL, "null argument");
+    CK(cudaSetDevice(c->device));
+    std::string err;
+    const int rc = ualm_fe::set_map(&c->fe, m, err);
+    return rc < 0 ? fail(rc, err) : rc;
+}
+
+extern "C" int ualm_front_end_batch_device(ualm_ctx_t *c, const ualm_astar_params_t *ap, const ualm_resample_params_t *rp, int B, const double *starts,
+                                           const double *goals, int32_t *N, int32_t *M, double *bnd, double *total_time, double *inner_xy,
+                                           long long cap_xy, double *inner_yaw, long long cap_yaw, int32_t *packed, int32_t *n_expanded,
+                                           double *path_xyyaw, long long cap_path, int64_t *path_off, float *search_ms)
+{
+    if (!c) return fail(UALM_EINVAL, "null ctx");
+    CK(cudaSetDevice(c->device));
+    std::string err;
+    const int rc = ualm_fe::batch(c->fe, ap, rp, B, starts, goals, N, M, bnd, total_time, inner_xy, cap_xy, inner_yaw, cap_yaw, packed, n_expanded,
+                                  path_xyyaw, cap_path, path_off, search_ms, err);
+    return rc < 0 ? fail(rc, err) : rc;
+}
+
+extern "C" int ualm_front_end_path_cap(const ualm_astar_params_t *ap, const ualm_resample_params_t *rp)
+{
+    if (!ap || !rp) return fail(UALM_EINVAL, "null argument");
+    return ualm_fe::path_cap(ap, rp);
 }
